@@ -2,6 +2,7 @@
 """Headline benchmark: greedy generate through ``DistributedModel`` on N B200s (pipeline-sharded), tokens/s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload qwen2.5-7b|qwen2.5-0.5b|...] [--impl reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -34,6 +35,7 @@ WORKLOADS = {
     "qwen3-8b": ("Qwen/Qwen3-8B", 32, 128, 1),
     "tiny": ("tiny-qwen2-d128", 16, 32, 1),
 }
+DUMP_LIMIT_BYTES = 64_000_000      # all of --dump-outputs, .npy headers included
 
 
 def measured_peaks():
@@ -50,6 +52,21 @@ def burst_tflops(default):
     if os.path.exists(p):
         return float(json.load(open(p)).get("bf16_tflops", default))
     return default
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as ``out_dir/<name>.npy`` in float64, so that two builds run with the same arguments can be
+    compared output for output.  An array larger than its share of DUMP_LIMIT_BYTES keeps a fixed, seeded sample of its
+    rows (the same rows on every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // len(arrays) - 4096
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > share:
+            keep = np.random.default_rng(0).choice(len(a), share // a[0].nbytes, replace=False)
+            a = a[np.sort(keep)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -527,7 +544,13 @@ def main():
     ap.add_argument("--train-batch", type=int, default=8)
     ap.add_argument("--train-seq", type=int, default=512)
     ap.add_argument("--train-mb-per-stage", type=int, default=4, help="micro-batches per pipeline stage in the training step (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the token ids the last timed generate "
+                                                          "returned as DIR/sequences.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 arm computed; the reference arm times a bounded CPU sample")
     name, prompt, new, wl_rows = WORKLOADS[args.workload]
     prompt, new = args.prompt or prompt, args.new or new
     args.rows_per_gpu = args.rows_per_gpu or wl_rows
@@ -634,6 +657,8 @@ def main():
     sync_all()
     t_e2e = torch.tensor([max(e2.elapsed_time(e3) * 1e-3, time.perf_counter() - t0)], device=dm.device)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"sequences": out_host.numpy()})
     # ---- pipeline occupancy: fraction of the decode phase this rank's compute stream spent inside decode launches
     # (the rest = waiting for a neighbour's activations / ids, i.e. exposed transfer + pipeline bubble)
     dm.generate(ids_dev, max_new_tokens=new, profile=True)

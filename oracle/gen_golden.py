@@ -2,6 +2,9 @@
 
 Run in the build container (needs /root/reference):  python -m oracle.gen_golden
 Writes tests/golden/ref_layergroup_<cfg>.pt (a few hundred KB each).
+``python -m oracle.gen_golden --portable`` writes tests/golden/ref_layergroup_eager_portable.json instead: SHA-256 of
+every hop and of the last-4 logits of the eager runs, computed with the host-independent CPU arithmetic of
+oracle/portable_cpu.py, so that tests/test_golden.py can check the oracle against them bit for bit on any x86-64 host.
 
 What runs, unmodified, from the reference:
   * ``tensorlink.ml.injector.LayerGroupModule`` (injector.py:154-281) executing the HF decoder-layer loop
@@ -12,10 +15,14 @@ reference pins; its own AST finder does not match transformers 5.x loops, SURVEY
 Layers are the installed HF ``Qwen2DecoderLayer``/``Qwen3DecoderLayer`` with the seeded weights; host-side
 embed / rotary / mask / final norm / lm_head are HF's (module.py:1023-1056 keeps them on the host).
 """
+import hashlib
+import json
 import os
+import sys
 
 import torch
 
+from oracle import portable_cpu
 from oracle.ref_shim import import_reference
 from tensorlink_b200.ml import configs as C
 from tensorlink_b200.ml.weights import init_state_dict, synthetic_tokens
@@ -68,9 +75,30 @@ def run(cfg, n_shards, B, S, attn, dtype=torch.bfloat16):
             "dtype": str(dtype)}
 
 
+CASES = ((C.TINY_QWEN2, 2, 2, 24), (C.TINY_QWEN3, 3, 1, 17), (C.TINY_QWEN2_D128, 2, 1, 33))
+
+
+def sha256_bf16(t):
+    return hashlib.sha256(t.contiguous().view(torch.int16).numpy().tobytes()).hexdigest()
+
+
+def portable():
+    if not portable_cpu.active():          # read when torch loads: start again with the variables set
+        os.execve(sys.executable, [sys.executable, "-m", "oracle.gen_golden", "--portable"], dict(os.environ, **portable_cpu.ENV))
+    portable_cpu.apply()
+    out = {}
+    for cfg, n, B, S in CASES:
+        g = run(cfg, n, B, S, "eager")
+        out[cfg.name] = {"hops_sha256": [sha256_bf16(h) for h in g["hops"]], "logits_sha256": sha256_bf16(g["logits"][:, -4:, :])}
+    path = os.path.join(OUT, "ref_layergroup_eager_portable.json")
+    with open(path, "w") as f:
+        json.dump(out, f, indent=1)
+    print(path)
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
-    for cfg, n, B, S in ((C.TINY_QWEN2, 2, 2, 24), (C.TINY_QWEN3, 3, 1, 17), (C.TINY_QWEN2_D128, 2, 1, 33)):
+    for cfg, n, B, S in CASES:
         for attn in ("eager", "sdpa"):
             g = run(cfg, n, B, S, attn)
             path = os.path.join(OUT, f"ref_layergroup_{cfg.name}_{attn}.pt")
@@ -81,4 +109,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    portable() if sys.argv[1:] == ["--portable"] else main()

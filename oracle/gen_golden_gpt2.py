@@ -9,13 +9,16 @@ ml/injector.py:75-90; SURVEY.md §8c), so the loop body is handed to LayerGroupM
 output equals the unsharded HF model BIT FOR BIT on CPU — the sharding + codec add no numeric change.  GPT-2 itself is
 not on the B200 path (LayerNorm / GELU / learned positions have no kernels here: config 1 is the reference's CPU
 plumbing case); tests/test_gpt2_plumbing_cpu.py re-runs the same 2-shard composition through THIS repo's wire codec
-(oracle and product) on CPU and checks it against the fixture written here.
+(oracle and product) on CPU and checks it against the fixture written here.  Both run with the host-independent CPU
+arithmetic of oracle/portable_cpu.py, so that the SHA-256 comparison holds on any x86-64 host.
 """
 import hashlib
 import os
+import sys
 
 import torch
 
+from oracle import portable_cpu
 from oracle.ref_shim import import_reference
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden", "ref_gpt2_2shards.pt")
@@ -55,6 +58,9 @@ def host_side(m, ids):
 
 
 def main():
+    if not portable_cpu.active():          # read when torch loads: start again with the variables set
+        os.execve(sys.executable, [sys.executable, "-m", "oracle.gen_golden_gpt2"], dict(os.environ, **portable_cpu.ENV))
+    portable_cpu.apply()
     injector, utils = import_reference()
     m, ids = gpt2_small(), tokens()
     with torch.no_grad():

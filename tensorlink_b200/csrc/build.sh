@@ -4,13 +4,19 @@ set -euo pipefail
 here="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
 out="$here/libtensorlink_b200.so"
 srcs=("$here"/*.cu)
+hdrs=("$here"/*.cuh "$here/../../include/tensorlink_b200.h")
 objs=()
 mkdir -p "$here/build"
 pids=()
+stale() {  # object $1 of source $2: missing, or older than the source or any header
+  [[ -f "$1" && ! "$2" -nt "$1" ]] || return 0
+  for h in "${hdrs[@]}"; do [[ "$h" -nt "$1" ]] && return 0; done
+  return 1
+}
 for s in "${srcs[@]}"; do
   o="$here/build/$(basename "${s%.cu}").o"
   objs+=("$o")
-  if [[ ! -f "$o" || "$s" -nt "$o" || "$here/common.cuh" -nt "$o" || "$here/../../include/tensorlink_b200.h" -nt "$o" ]]; then
+  if stale "$o" "$s"; then
     nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC \
          ${TL_NVCC_EXTRA:-} -c "$s" -o "$o" &
     pids+=($!)

@@ -1,4 +1,8 @@
-"""Run under torchrun (gloo, CPU): exercises DistributedModel's multi-rank host logic with the oracle stage."""
+"""Run under torchrun (gloo, CPU): exercises DistributedModel's multi-rank host logic with the oracle stage.
+
+Started with the host-independent CPU arithmetic of oracle/portable_cpu.py: the pipelined results are compared bit for bit
+with one unsharded oracle run, and with the default ISA-specific kernels the two ways of blocking the same math round
+differently on some CPUs."""
 import os
 import sys
 
@@ -7,6 +11,7 @@ import torch.distributed as dist
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+from oracle import portable_cpu  # noqa: E402
 from oracle import shard_oracle as O  # noqa: E402
 from tensorlink_b200.ml import DistributedModel  # noqa: E402
 from tensorlink_b200.ml import configs as C  # noqa: E402
@@ -16,7 +21,7 @@ from tests.oracle_stage import OracleStage  # noqa: E402
 
 
 def main(out_dir):
-    torch.set_num_threads(2)
+    portable_cpu.apply()
     init_process_group_from_env("gloo")
     rank, world = dist.get_rank(), dist.get_world_size()
     cfg = C.TINY_QWEN2_D128
@@ -26,7 +31,7 @@ def main(out_dir):
     # 1) inference forward with logits gathered to rank 0, and the plan handed in explicitly (reference schema)
     from tensorlink_b200.ml import graphing
     plan = graphing.make_plan(cfg, world)
-    dm = DistributedModel(cfg, training=False, config=plan, max_batch=4, max_seq=64, _stage_factory=OracleStage)
+    dm = DistributedModel(cfg, training=False, config=plan, max_batch=4, max_seq=64, _stage_factory=OracleStage, device="cpu")
     ids = synthetic_tokens(cfg, 2, 12)
     out = dm(ids if rank == 0 else None, gather_logits=True)
     if rank == 0:
@@ -51,7 +56,7 @@ def main(out_dir):
             self.ended = True
     st = Streamer()
     gen = dm.generate(ids if rank == 0 else None, max_new_tokens=6, streamer=st)
-    dm2 = DistributedModel(cfg, training=False, n_pipelines=2, max_batch=4, max_seq=64, _stage_factory=OracleStage)
+    dm2 = DistributedModel(cfg, training=False, n_pipelines=2, max_batch=4, max_seq=64, _stage_factory=OracleStage, device="cpu")
     ids4 = synthetic_tokens(cfg, 4, 9)
     gen2 = dm2.generate(ids4 if rank == 0 else None, max_new_tokens=5)
     ref_gen = O.OracleModel(cfg, sd, "sdpa_math").generate(ids, 6)
@@ -88,7 +93,7 @@ def main(out_dir):
     res["left_pad_ok"] = ok
     # a batch the requested micro-batch count does not divide (3 rows, n_pipelines = 2 -> one micro-batch of 3 rows)
     ids3 = synthetic_tokens(cfg, 3, 7, seed=77)
-    dm3 = DistributedModel(cfg, training=False, n_pipelines=2, max_batch=6, max_seq=64, _stage_factory=OracleStage)
+    dm3 = DistributedModel(cfg, training=False, n_pipelines=2, max_batch=6, max_seq=64, _stage_factory=OracleStage, device="cpu")
     gen3 = dm3.generate(ids3 if rank == 0 else None, max_new_tokens=4)
     res["odd_batch_ok"] = bool(torch.equal(gen3, O.OracleModel(cfg, sd, "sdpa_math").generate(ids3, 4)))
     # streamer + early stop: the callback sees exactly the columns the (stopped) loop produced, then end()
@@ -103,7 +108,7 @@ def main(out_dir):
     if rank == 0:
         res["stream_ok"] = st.ended and torch.equal(torch.stack(st.cols, 1), ref_gen[:, 12:])
     # 3) training step: loss on every rank, backward through the ranks, grads match single-process autograd
-    dmt = DistributedModel(cfg, training=True, n_pipelines=2, max_batch=4, max_seq=64, _stage_factory=OracleStage,
+    dmt = DistributedModel(cfg, training=True, n_pipelines=2, max_batch=4, max_seq=64, _stage_factory=OracleStage, device="cpu",
                            optimizer=torch.optim.Adam)
     tids = synthetic_tokens(cfg, 4, 16)
     o = dmt(tids if rank == 0 else None, labels=tids if rank == 0 else None)
@@ -123,7 +128,7 @@ def main(out_dir):
     # embedding gradient + lm_head gradient = the single-process gradient of the shared tensor
     tcfg = C.TINY_QWEN2
     tsd = init_state_dict(tcfg)
-    dtie = DistributedModel(tcfg, training=True, n_pipelines=2, max_batch=4, max_seq=64, _stage_factory=OracleStage,
+    dtie = DistributedModel(tcfg, training=True, n_pipelines=2, max_batch=4, max_seq=64, _stage_factory=OracleStage, device="cpu",
                             optimizer=torch.optim.Adam)
     tt = synthetic_tokens(tcfg, 4, 12)
     dtie(tt if rank == 0 else None, labels=tt if rank == 0 else None).loss.backward()

@@ -9,6 +9,8 @@ import sys
 import pytest
 import torch
 
+from oracle import portable_cpu
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -22,7 +24,7 @@ def _free_port():
 def test_pipeline_host_logic(tmp_path, world):
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}", "--master-addr", "127.0.0.1",
            "--master-port", str(_free_port()), os.path.join(ROOT, "tests", "pipeline_worker.py"), str(tmp_path)]
-    env = dict(os.environ, OMP_NUM_THREADS="2", PYTHONPATH=ROOT)
+    env = dict(os.environ, PYTHONPATH=ROOT, **portable_cpu.ENV)
     r = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=900)
     errs = "".join(open(p).read() for p in sorted(map(str, tmp_path.glob("err*.txt"))))
     assert r.returncode == 0, errs or r.stderr[-3000:]
