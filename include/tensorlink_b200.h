@@ -238,8 +238,11 @@ int tl_attn_bwd(const void* q, const void* k_cache, const void* v_cache, const v
  * with a valid label; dlogits = (softmax - onehot) * grad_scale (may alias logits); label outside [0,V) ignored */
 int tl_ce_fwd_bwd(const void* logits, const int64_t* labels, float* loss_sum, int32_t* n_valid, void* dlogits,
                   float grad_scale, int M, int V, void* stream);
-/* embedding backward: dtable[ids[n],:] += dout[n,:]  (bf16x2 atomics into the bf16 gradient) */
-int tl_embed_bwd(const int64_t* ids, const void* dout, void* dtable, int n_tokens, int H, int vocab, void* stream);
+/* embedding backward: dtable[id,:] += sum of dout[n,:] over the tokens n with ids[n] == id, summed in fp32 in token
+ * order and rounded once into the bf16 row (deterministic, no atomics).  Takes the ids stably sorted (sorted_ids) and
+ * the token index of each (order); ids outside [0, vocab) are skipped.  H %% 8 == 0, dout / dtable 16-byte aligned */
+int tl_embed_bwd(const int64_t* sorted_ids, const int64_t* order, const void* dout, void* dtable, int n_tokens, int H,
+                 int vocab, void* stream);
 /* bias gradient: db_accum[N] (fp32) += sum_m dy[m,:N] (row pitch ld) */
 int tl_colsum(const void* dy, float* db_accum, int M, int N, int ld, void* stream);
 /* dst[n] (+)= src[n]: fp32 accumulator into a bf16 gradient */

@@ -382,15 +382,52 @@ __global__ void __launch_bounds__(CE_THREADS) ce_fwd_bwd_kernel(const bf16* __re
 }
 
 // ------------------------------------------------------------------------------------------------ embedding backward
-__global__ void embed_bwd_kernel(const int64_t* __restrict__ ids, const bf16* __restrict__ dout, bf16* __restrict__ dtable,
-                                 int n_tokens, int H, int vocab) {
-    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (warp >= n_tokens) return;
-    const long long id = ids[warp];
-    if (id < 0 || id >= vocab) return;
-    const __nv_bfloat162* src = reinterpret_cast<const __nv_bfloat162*>(dout + (size_t)warp * H);
-    __nv_bfloat162* dst = reinterpret_cast<__nv_bfloat162*>(dtable + (size_t)id * H);
-    for (int i = lane; i < (H >> 1); i += 32) atomicAdd(&dst[i], src[i]);
+// ids arrive stably sorted, order[i] = the token holding sorted_ids[i].  The CTAs at the first position of a run of
+// equal ids (blockIdx.y: 8-column vectors) sum the run's gradient rows in fp32, in token order, and add the sum to the
+// bf16 table row with one rounding.  No atomics: the result is deterministic, and an id that occurs k times is rounded
+// once instead of k times (bf16 atomics: rel-L2 2e-2 at k = 256).  A heavy id is summed by H/512 CTAs alone.
+constexpr int EB_THREADS = 64, EB_BATCH = 16;
+__global__ void __launch_bounds__(EB_THREADS) embed_bwd_kernel(const int64_t* __restrict__ sorted_ids,
+                                                               const int64_t* __restrict__ order, const bf16* __restrict__ dout,
+                                                               bf16* __restrict__ dtable, int n_tokens, int H, int vocab) {
+    const int i0 = blockIdx.x;
+    const long long id = sorted_ids[i0];
+    if (id < 0 || id >= vocab || (i0 > 0 && sorted_ids[i0 - 1] == id)) return;
+    // end of the run, 32 positions per step (each warp finds the same end)
+    const int lane = threadIdx.x & 31;
+    int i1 = i0 + 1;
+    for (;;) {
+        const int i = i1 + lane;
+        const unsigned stop = __ballot_sync(0xffffffffu, i >= n_tokens || sorted_ids[i] != id);
+        if (stop) { i1 += __ffs(stop) - 1; break; }
+        i1 += 32;
+    }
+    const int c = blockIdx.y * EB_THREADS + threadIdx.x;
+    if (c >= (H >> 3)) return;
+    float acc[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) acc[j] = 0.f;
+    for (int i = i0; i < i1; i += EB_BATCH) {
+        const int nb = min(EB_BATCH, i1 - i);
+        uint4 r[EB_BATCH];
+#pragma unroll
+        for (int j = 0; j < EB_BATCH; ++j)          // all loads of the batch in flight before the first add
+            if (j < nb) r[j] = reinterpret_cast<const uint4*>(dout + (size_t)order[i + j] * H)[c];
+#pragma unroll
+        for (int j = 0; j < EB_BATCH; ++j) {
+            if (j < nb) {
+                const uint32_t* p = reinterpret_cast<const uint32_t*>(&r[j]);
+#pragma unroll
+                for (int q = 0; q < 4; ++q) { acc[2 * q] += bf16_lo(p[q]); acc[2 * q + 1] += bf16_hi(p[q]); }
+            }
+        }
+    }
+    uint4* dst = reinterpret_cast<uint4*>(dtable + (size_t)id * H) + c;
+    uint4 t = *dst;
+    uint32_t* t32 = reinterpret_cast<uint32_t*>(&t);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) t32[q] = pack_bf16(bf16_lo(t32[q]) + acc[2 * q], bf16_hi(t32[q]) + acc[2 * q + 1]);
+    *dst = t;
 }
 
 // ------------------------------------------------------------------------------------------------ column sum (bias grad)
@@ -630,11 +667,15 @@ int tl_ce_fwd_bwd(const void* logits, const int64_t* labels, float* loss_sum, in
     return check_launch("tl_ce_fwd_bwd");
 }
 
-int tl_embed_bwd(const int64_t* ids, const void* dout, void* dtable, int n_tokens, int H, int vocab, void* stream) {
+int tl_embed_bwd(const int64_t* sorted_ids, const int64_t* order, const void* dout, void* dtable, int n_tokens, int H, int vocab,
+                 void* stream) {
     using namespace tl;
-    TL_REQUIRE(H % 2 == 0, TL_ERR_INVALID, "tl_embed_bwd: H odd");
+    TL_REQUIRE(H % 8 == 0 && H > 0, TL_ERR_INVALID, "tl_embed_bwd: H %% 8 != 0 (H=%d)", H);
+    TL_REQUIRE(((((uintptr_t)dout) | ((uintptr_t)dtable)) & 15) == 0, TL_ERR_INVALID, "tl_embed_bwd: 16-byte alignment required");
     if (n_tokens == 0) return TL_OK;
-    embed_bwd_kernel<<<(n_tokens + 7) / 8, 256, 0, (cudaStream_t)stream>>>(ids, (const bf16*)dout, (bf16*)dtable, n_tokens, H, vocab);
+    const dim3 grid(n_tokens, (H / 8 + EB_THREADS - 1) / EB_THREADS);
+    embed_bwd_kernel<<<grid, EB_THREADS, 0, (cudaStream_t)stream>>>(sorted_ids, order, (const bf16*)dout, (bf16*)dtable, n_tokens,
+                                                                     H, vocab);
     return check_launch("tl_embed_bwd");
 }
 

@@ -77,7 +77,7 @@ _SIGS = {
     "tl_attn_bwd_ws": (c_size_t, [c_int, c_int, c_int]),
     "tl_attn_bwd": (c_int, [c_void_p] * 10 + [c_size_t, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p]),
     "tl_ce_fwd_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_int, c_int, c_void_p]),
-    "tl_embed_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "tl_embed_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "tl_colsum": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "tl_f32_to_bf16_accum": (c_int, [c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
     "tl_add_inplace": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p]),
@@ -439,6 +439,13 @@ def rmsnorm_bwd(x, w, dy, rstd, dx, dw_accum, dx_add=None):
 
 
 def rope_kv_bwd(dq, dk, dv, dqkv, cos_tab, sin_tab, S, n_h, n_kv, d):
+    # the kernel takes T_max from dk and indexes every buffer from these sizes: a mismatch would read or write out of bounds
+    n_tokens = dqkv.shape[0]
+    assert n_tokens % S == 0 and tuple(dqkv.shape) == (n_tokens, (n_h + 2 * n_kv) * d), (tuple(dqkv.shape), S, n_h, n_kv, d)
+    assert dq.numel() == n_tokens * n_h * d, (tuple(dq.shape), n_tokens, n_h, d)
+    assert tuple(dk.shape) == tuple(dv.shape) == (n_tokens // S, n_h, dk.shape[2], d) and dk.shape[2] >= S, \
+        (tuple(dk.shape), tuple(dv.shape), S, n_h, d)
+    assert cos_tab.shape == sin_tab.shape and cos_tab.shape[0] >= S and cos_tab.shape[1] == d // 2, (tuple(cos_tab.shape), S, d)
     require_device(); _bf16(dq, dk, dv, dqkv)
     _check(load().tl_rope_kv_bwd(_p(dq), _p(dk), _p(dv), _p(dqkv), _p(cos_tab), _p(sin_tab), dqkv.shape[0], S, n_h, n_kv,
                                  d, dk.shape[2], _stream()), "tl_rope_kv_bwd")
@@ -449,9 +456,17 @@ def attn_bwd_ws(B, S, n_h) -> int:
 
 
 def attn_bwd(q, k_cache, v_cache, out, dout, lse, dq, dk, dv, ws, B, S, n_h, n_kv, d, scale):
+    # T_max comes from k_cache and is also the row pitch of dk / dv: their shapes must agree with it
+    T_max = k_cache.shape[2]
+    assert tuple(k_cache.shape) == tuple(v_cache.shape) == (B, n_kv, T_max, d) and S <= T_max, \
+        (tuple(k_cache.shape), tuple(v_cache.shape), B, S, n_kv, d)
+    assert tuple(dk.shape) == tuple(dv.shape) == (B, n_h, T_max, d), (tuple(dk.shape), tuple(dv.shape), B, n_h, T_max, d)
+    n = B * S * n_h * d
+    assert q.numel() == out.numel() == dout.numel() == dq.numel() == n and lse.numel() == B * n_h * S, \
+        (tuple(q.shape), tuple(out.shape), tuple(dout.shape), tuple(dq.shape), tuple(lse.shape), B, S, n_h, d)
     require_device(); _bf16(q, k_cache, v_cache, out, dout, dq, dk, dv)
     _check(load().tl_attn_bwd(_p(q), _p(k_cache), _p(v_cache), _p(out), _p(dout), _p(lse), _p(dq), _p(dk), _p(dv), _p(ws),
-                              ws.numel() * ws.element_size(), B, S, n_h, n_kv, d, k_cache.shape[2], scale, _stream()),
+                              ws.numel() * ws.element_size(), B, S, n_h, n_kv, d, T_max, scale, _stream()),
            "tl_attn_bwd")
 
 
@@ -464,9 +479,15 @@ def ce_fwd_bwd(logits, labels, loss_sum, n_valid, dlogits, grad_scale: float):
 
 
 def embed_bwd(ids, dout, dtable):
-    require_device(); _bf16(dout, dtable)
+    """dtable[id] += the fp32 sum of dout's rows of the tokens holding id, rounded once (deterministic); ids outside
+    [0, V) are skipped."""
     V, H = dtable.shape
-    _check(load().tl_embed_bwd(_p(ids), _p(dout), _p(dtable), ids.numel(), H, V, _stream()), "tl_embed_bwd")
+    n = ids.numel()
+    assert ids.dtype == torch.int64, ids.dtype
+    assert dout.shape[-1] == H and dout.numel() == n * H, (tuple(dout.shape), n, H)
+    require_device(); _bf16(dout, dtable)
+    sorted_ids, order = torch.sort(ids.reshape(-1), stable=True)     # one run per distinct id, tokens in order
+    _check(load().tl_embed_bwd(_p(sorted_ids), _p(order), _p(dout), _p(dtable), n, H, V, _stream()), "tl_embed_bwd")
 
 
 def colsum(dy, db_accum):
